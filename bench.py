@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the non-key-frame propagation + aggregation path (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   torchrun --nproc-per-node N ... bench.py --gpus N ...      (one rank per GPU, no collective
                                                               on the data path: streams shard)
 
@@ -17,6 +17,10 @@ One "step" = one pass of the hot path over one batch of synthetic frames:
 `cpu_baseline`: the reference's CPU path (C port of the MXNet CPU operators, oracle/) timed on
            this box's host cores on a bounded sample.
 `--impl reference` times that CPU path alone and prints the same line with "impl":"reference".
+`--dump-outputs DIR` (rank 0): after the timed steps, what each timed path returned in its last step -
+           value.npy (the device output), e2e.npy and e2e_gop.npy (the host output of the two e2e rows) - as
+           float32, each a fixed seeded sample of DUMP_SAMPLE values when the output is larger.  The inputs are
+           seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -42,6 +46,20 @@ def algorithmic_bytes_v2(frames, feat_bytes=4):
     """SURVEY.md 8d, V2: 4F (key, scale, cur, out) + 32*HW (4 MV taps x 2 ch x 4 B) + 8*HW (logits)."""
     F = C * H * W * feat_bytes
     return frames * (4 * F + 32 * H * W + 8 * H * W)
+
+
+DUMP_SAMPLE = 4 << 20             # values per dumped output: 3 x 16 MB stays within 64 MB
+
+
+def dump_sample(t):
+    """float32 numpy copy of `t` (device or host tensor), or of DUMP_SAMPLE of its values when it is larger: flat indices
+    drawn with a fixed seed and sorted, so every run with the same output shape samples the same elements."""
+    import numpy as np
+    import torch
+    if t.numel() <= DUMP_SAMPLE:
+        return t.float().cpu().numpy()
+    idx = np.sort(np.random.default_rng(0).integers(0, t.numel(), DUMP_SAMPLE))
+    return t.reshape(-1)[torch.from_numpy(idx).to(t.device)].float().cpu().numpy()
 
 
 def workload_config(frames, n_gpus):
@@ -324,6 +342,9 @@ def run_ours(args):
     value = total_frames / (ms / 1e3)
     launches = K * prep.launches
     clocks = sampler.summary()
+    dumps = {} if args.dump_outputs is not None and rank == 0 else None
+    if dumps is not None:
+        dumps["value"] = dump_sample(prep.out)
 
     # roofline of the dominant (only) kernel: algorithmic bytes per launch / launch duration
     peak, peak_src = measured_hbm_peak()
@@ -376,6 +397,8 @@ def run_ours(args):
         return gather_frame_counts(frames * steps, ms_l)
 
     e2e_frames, e2e_ms = time_host_path(agg, host, e2e_steps)
+    if dumps is not None:
+        dumps["e2e"] = dump_sample(out_host)
     bi, bo = agg.bytes_per_call()
     e2e_gbs = world * (bi + bo) * e2e_steps / (e2e_ms / 1e3) / 1e9
     e2e = {"value": e2e_frames / (e2e_ms / 1e3), "unit": UNIT, "h2d_bytes_per_step": bi, "d2h_bytes_per_step": bo,
@@ -400,6 +423,8 @@ def run_ours(args):
     host_g["new_keys"] = host["key"][:n_keys]
     host_g["key_slot"] = torch.arange(n_keys, dtype=torch.int32).pin_memory()
     g_frames, g_ms = time_host_path(agg_g, host_g, e2e_steps)
+    if dumps is not None:
+        dumps["e2e_gop"] = dump_sample(out_host)
     gbi, gbo = agg_g.bytes_per_call(host_g)
     g_gbs = world * (gbi + gbo) * e2e_steps / (g_ms / 1e3) / 1e9
     e2e["gop_contract"] = {"value": g_frames / (g_ms / 1e3), "unit": UNIT, "h2d_bytes_per_step": gbi, "d2h_bytes_per_step": gbo,
@@ -442,6 +467,11 @@ def run_ours(args):
         }
         if extra:
             line["extra"] = extra
+        if dumps is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, a in dumps.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), a)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -463,7 +493,8 @@ def time_launches(fn, warmup, steps):
 
 
 def run_extras(dev, d, args):
-    """Secondary numbers (never the headline): bf16 NHWC variant, unfused ablation, hi-res config."""
+    """Secondary numbers (never the headline): bf16 NHWC variant, unfused ablation, hi-res config.  They time their own
+    step counts (--steps capped at 20, or fixed per row), recorded as each row's "steps"."""
     import torch
 
     from lsfa_b200 import ops
@@ -476,7 +507,8 @@ def run_extras(dev, d, args):
         flow = ops.mv_pool(d["mv"])
         tmp = torch.empty(5 * d["key"].numel(), dtype=torch.float32, device=dev)
         ms_u = time_launches(lambda: ops.unfused_chain(d["key"], flow, d["scale_map"], d["cur"], d["logits"], tmp), 3, steps)
-        out["unfused_fp32_nchw"] = {"frames_per_s": frames / (ms_u / 1e3), "ms_per_step": ms_u, "launches_per_step": 9}
+        out["unfused_fp32_nchw"] = {"frames_per_s": frames / (ms_u / 1e3), "ms_per_step": ms_u, "launches_per_step": 9,
+                                    "steps": steps}
         del tmp
     except Exception as e:
         out["unfused_fp32_nchw"] = {"error": repr(e)}
@@ -488,7 +520,7 @@ def run_extras(dev, d, args):
         ms_p = time_launches(lambda: prep2.run(s2), 3, steps)
         gb = algorithmic_bytes_v2(frames, 4) / (ms_p / 1e3) / 1e9
         out["fused_fp32_nchw_plane_ldg"] = {"frames_per_s": frames / (ms_p / 1e3), "ms_per_step": ms_p,
-                                            "achieved_gbs": gb, "frac_of_measured_peak": gb / peak}
+                                            "achieved_gbs": gb, "frac_of_measured_peak": gb / peak, "steps": steps}
     except Exception as e:
         out["fused_fp32_nchw_plane_ldg"] = {"error": repr(e)}
     try:
@@ -500,7 +532,7 @@ def run_extras(dev, d, args):
         ms_b = time_launches(lambda: prep.run(s), 3, steps)
         gb = algorithmic_bytes_v2(frames, 2) / (ms_b / 1e3) / 1e9
         out["fused_bf16_nhwc"] = {"frames_per_s": frames / (ms_b / 1e3), "ms_per_step": ms_b, "achieved_gbs": gb,
-                                  "frac_of_measured_peak": gb / peak}
+                                  "frac_of_measured_peak": gb / peak, "steps": steps}
         # BASELINE configs[2] proper: the same in bf16 channels-last at batch 512 (the resident frames tiled 512/frames times)
         reps = max(1, 512 // frames)
         if reps > 1:
@@ -512,7 +544,7 @@ def run_extras(dev, d, args):
             nb = frames * reps
             gb = algorithmic_bytes_v2(nb, 2) / (ms_c / 1e3) / 1e9
             out["fused_bf16_nhwc_batch512"] = {"frames": nb, "frames_per_s": nb / (ms_c / 1e3), "ms_per_step": ms_c,
-                                               "achieved_gbs": gb, "frac_of_measured_peak": gb / peak}
+                                               "achieved_gbs": gb, "frac_of_measured_peak": gb / peak, "steps": min(steps, 10)}
             del big, prep
         nf = {k: ops.to_nhwc(d[k], torch.float32) for k in ("key", "cur", "scale_map")}
         prep = ops.PreparedAggregate(nf["key"], d["mv"], flow_kind="raw", cur=nf["cur"], scale_map=nf["scale_map"],
@@ -520,7 +552,7 @@ def run_extras(dev, d, args):
         ms_f = time_launches(lambda: prep.run(s), 3, steps)
         gb = algorithmic_bytes_v2(frames, 4) / (ms_f / 1e3) / 1e9
         out["fused_fp32_nhwc"] = {"frames_per_s": frames / (ms_f / 1e3), "ms_per_step": ms_f, "achieved_gbs": gb,
-                                  "frac_of_measured_peak": gb / peak}
+                                  "frac_of_measured_peak": gb / peak, "steps": steps}
     except Exception as e:
         out["fused_bf16_nhwc"] = {"error": repr(e)}
     for name, fn in (("cfg1_single_frame", extra_cfg1), ("cfg4_hires_68x120", extra_cfg4), ("cfg5_multi_stream", extra_cfg5),
@@ -545,7 +577,7 @@ def extra_cfg1(dev, d, peak, steps):
     s = torch.cuda.current_stream().cuda_stream
     grid = torch.empty((1, 2, H, W), device=dev)
     o = torch.empty_like(key)
-    r = {}
+    r = {"steps": 200}                  # per timing below
     ms = time_launches(lambda: ops.BilinearSampler(key, ops.GridGenerator(ops.mv_pool(mv), out=grid), out=o), 10, 200)
     r["three_dropin_operators_us"] = 1e3 * ms
     p0 = ops.PreparedAggregate(key, mv, flow_kind="raw")
@@ -614,7 +646,8 @@ def extra_cfg4(dev, d, peak, steps):
         ms = time_launches(lambda: prep.run(s), 3, min(steps, 10))
         alg = N4 * (4 * C * H4 * W4 * fb + 40 * H4 * W4)
         gb = alg / (ms / 1e3) / 1e9
-        r[tag] = {"frames": N4, "frames_per_s": N4 / (ms / 1e3), "ms_per_step": ms, "achieved_gbs": gb, "frac_of_measured_peak": gb / peak}
+        r[tag] = {"frames": N4, "frames_per_s": N4 / (ms / 1e3), "ms_per_step": ms, "achieved_gbs": gb, "frac_of_measured_peak": gb / peak,
+                  "steps": min(steps, 10)}
         del key, cur, sm, prep
         torch.cuda.empty_cache()
     return r
@@ -655,7 +688,7 @@ def extra_cfg5(dev, d, peak, steps):
     fps = frames / (ms / 1e3)
     return {"streams": S, "frames_per_step": frames, "launches_per_step": len(slots), "ms_per_step": ms, "frames_per_s": fps,
             "alg_bytes_per_frame": alg, "achieved_gbs": fps * alg / 1e9, "frac_of_measured_peak": fps * alg / 1e9 / peak,
-            "key_table_gb": sch.key_table.numel() * 4 / 1e9}
+            "key_table_gb": sch.key_table.numel() * 4 / 1e9, "steps": 5}
 
 
 def extra_backward(dev, d, peak, steps):
@@ -678,7 +711,7 @@ def extra_backward(dev, d, peak, steps):
             ("fused_v2_backward_all_gradients", lambda: ops.warp_scale_aggregate_backward(og, d["key"], flow, flow_kind="flow", cur=d["cur"], scale_map=d["scale_map"], weight_mode="logits", logits=d["logits"]), 10 * F4)):
         ms = time_launches(fn, 2, 10)
         gb = n * alg / (ms / 1e3) / 1e9
-        r[tag] = {"ms_per_step": ms, "frames_per_s": n / (ms / 1e3), "achieved_gbs": gb, "frac_of_measured_peak": gb / peak}
+        r[tag] = {"ms_per_step": ms, "frames_per_s": n / (ms / 1e3), "achieved_gbs": gb, "frac_of_measured_peak": gb / peak, "steps": 10}
     return r
 
 
@@ -711,13 +744,15 @@ def extra_keyframe(dev, d, peak, steps):
     r = {"key_frames": N, "tensor_peak_tflops": tf_peak, "tensor_peak_source": tf_src}
     ms = time_launches(lambda: ops.embed_cosine_logits(xn, pe), 3, 10)
     r["embed_cosine_tcgen05"] = {"ms": ms, "gflop": gf_emb, "tflops": gf_emb / ms, "frac_of_sustained_bf16_peak": gf_emb / ms / tf_peak,
-                                 "launches": 4, "writes_embeddings": False}
+                                 "launches": 4, "writes_embeddings": False, "steps": 10}
     ms = time_launches(lambda: ops.nq_logits(xn, pq), 3, 10)
-    r["nq_tcgen05"] = {"ms": ms, "gflop": gf_nq, "tflops": gf_nq / ms, "frac_of_sustained_bf16_peak": gf_nq / ms / tf_peak, "launches": 1}
+    r["nq_tcgen05"] = {"ms": ms, "gflop": gf_nq, "tflops": gf_nq / ms, "frac_of_sustained_bf16_peak": gf_nq / ms / tf_peak, "launches": 1,
+                       "steps": 10}
     ms = time_launches(lambda: graphs.embed_net(xb, *embb), 2, 5)
-    r["embed_convs_cudnn_bf16"] = {"ms": ms, "tflops": gf_emb / ms, "note": "library arm: convolutions only, embeddings written to HBM, cosine not included"}
+    r["embed_convs_cudnn_bf16"] = {"ms": ms, "tflops": gf_emb / ms, "note": "library arm: convolutions only, embeddings written to HBM, cosine not included",
+                                   "steps": 5}
     ms = time_launches(lambda: graphs.nq_net(xb, *nqb), 2, 5)
-    r["nq_convs_cudnn_bf16"] = {"ms": ms, "tflops": gf_nq / ms}
+    r["nq_convs_cudnn_bf16"] = {"ms": ms, "tflops": gf_nq / ms, "steps": 5}
     return r
 
 
@@ -732,7 +767,11 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=0, help="0 = same as --steps")
     ap.add_argument("--no-extra", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (float32, sampled; --impl ours, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     return run_ours(args)

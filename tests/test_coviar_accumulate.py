@@ -51,7 +51,8 @@ def test_reconstruction_identity_of_the_reference():
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("algo", ["auto", "field", "trace"])
-@pytest.mark.parametrize("N,T,h,w", [(1, 1, 32, 48), (3, 4, 48, 80), (2, 11, 96, 160), (2, 3, 45, 77)])
+@pytest.mark.parametrize("N,T,h,w", [(1, 1, 32, 48), (3, 4, 48, 80), (2, 11, 96, 160), (2, 3, 45, 77),
+                                     (1, 11, 720, 1280)])       # a full-size GOP: 11 P-frames at 720p
 def test_gpu_mv_accumulate_bit_exact(cuda, N, T, h, w, algo):
     import torch
     from lsfa_b200 import ops
