@@ -271,6 +271,20 @@ LSFA_API size_t lsfa_cosine_logits_workspace_bytes(int N, int E, int H, int W, i
 LSFA_API int lsfa_cosine_logits_ws(const void* emb_warp, const void* emb_cur, float* logits, int N, int E, int H, int W,
                                    int layout, void* workspace, size_t workspace_bytes, void* stream);
 
+/* Backward of the NCHW float32 cosine logits (lsfa_cosine_logits_ws): from grad_logits (N,2,H,W) = d/d(logits) to
+ * grad_emb_warp, grad_emb_cur (N,E,H,W).  The logits are recomputed with the forward's kernel and summation order
+ * (the all-TMA pre-pass where lsfa_cosine_logits_ws with its full workspace runs it, else the LDG kernel), then one
+ * pass over both embeddings writes both gradients; no atomics, the results are the same bits run to run.
+ * req_* follow OpReqType (kNullOp or a NULL pointer skips that gradient).  The gradients must not overlap the inputs
+ * or each other.  workspace: lsfa_cosine_logits_backward_workspace_bytes, 16-byte aligned, no initialisation needed.
+ * kernel: 0 auto, 1 the plain LDG/STG kernel, 2 the all-TMA kernel (LSFA_E_UNSUPPORTED where it cannot serve the
+ * arguments: planes above 4,320 pixels, odd E or H*W, pointers not 16-byte aligned).  Both give the same bits. */
+LSFA_API size_t lsfa_cosine_logits_backward_workspace_bytes(int N, int E, int H, int W);
+LSFA_API int lsfa_cosine_logits_backward_f32_nchw(const float* emb_warp, const float* emb_cur, const float* grad_logits,
+                                                  float* grad_emb_warp, float* grad_emb_cur, int N, int E, int H, int W,
+                                                  int req_warp, int req_cur, void* workspace, size_t workspace_bytes,
+                                                  int kernel, void* stream);
+
 /* The reference graph op by op (one kernel per MXNet operator, each a full pass over
  * HBM) - the "unfused" arm of the ablation; same results as the fused op in LOGITS mode
  * with scale_map.  tmp: 5 feature-sized float32 buffers (N*C*H*W each), caller-owned. */
@@ -376,16 +390,23 @@ LSFA_API int lsfa_nq_logits_bf16_nhwc(const void* x, const void* w1, const float
 
 /* ---- backward of the fused operator's tails (SURVEY.md 8f rank 4; get_train_symbol SYM:306-338) -------------
  * Gradients of  out = wc*cur + ww*( BilinearSampler(key, GridGenerator(flow)) * scale_map + rnet_conv0(res) ),
- * (ww,wc) by weight_mode (NONE | ADD | MEAN | LOGITS = 2-way softmax), bypass frames: out = cur, with respect to every
+ * (ww,wc) by weight_mode (NONE | ADD | MEAN | LOGITS = 2-way softmax | COSINE = softmax of the cosine logits), bypass
+ * frames: out = cur, with respect to every
  * differentiable input, from d/d(out).  `fwd` is the forward's argument block (layout NCHW float32; `out` is not read
  * and may be any non-NULL pointer); each gradient has an OpReqType (NULL pointer or LSFA_REQ_NULL skips it).
  *   grad_key   (N,C,H,W)   needs private keys (key_index NULL) and key planes of the output's size
  *   grad_flow  (N,2,H,W)   LSFA_FLOW_PREPOOLED (flow in feature cells) or LSFA_FLOW_GRID (then it is d/d(grid));
  *                          raw motion vectors are integer data and get no gradient (SYM:319-321: the MV is data)
  *   grad_scale, grad_cur (N,C,H,W); grad_logits (N,2,H,W); grad_res (N,3,H,W); grad_rnet_w (C,3), grad_rnet_b (C)
+ *   grad_emb_warp, grad_emb_cur (N,E,H,W)   LSFA_W_COSINE only (one req_emb for both; a NULL pointer skips one).  The
+ *                          backward recomputes the cosine logits as the forward computes them with its full workspace
+ *                          (with force_generic == 1: as the LDG pre-pass does), runs the LOGITS-mode backward on them
+ *                          and then lsfa_cosine_logits_backward_f32_nchw.  grad_logits is not an output in this mode.
  * One pass over the feature streams (agg_tail_backward_kernel) + the a7/a8 gather backward for key/flow; every
- * reduction is summed in a fixed order (deterministic).  LSFA_W_COSINE has no backward here (its embeddings are inputs
- * of this library, produced by convolutions outside it).  workspace: the _workspace_bytes query, 256-byte aligned. */
+ * reduction is summed in a fixed order (deterministic).  Bypass frames get zero embedding gradients (req = write) or
+ * leave them untouched (req = add).  workspace: the _workspace_bytes query, 256-byte aligned.
+ * struct_bytes may also be the size of the struct before the embedding fields, offsetof(LsfaAggGrads, grad_emb_warp):
+ * those fields then read as NULL. */
 typedef struct LsfaAggGrads {
   int32_t struct_bytes;        /* = sizeof(LsfaAggGrads) */
   const float* out_grad;       /* (N,C,H,W) */
@@ -397,6 +418,7 @@ typedef struct LsfaAggGrads {
   float* grad_res;    int32_t req_res;
   float* grad_rnet_w; float* grad_rnet_b; int32_t req_rnet;
   void*  workspace;   size_t workspace_bytes;
+  float* grad_emb_warp; float* grad_emb_cur; int32_t req_emb;
 } LsfaAggGrads;
 LSFA_API size_t lsfa_warp_scale_aggregate_backward_workspace_bytes(const LsfaAggArgs* fwd, const LsfaAggGrads* grads);
 LSFA_API int    lsfa_warp_scale_aggregate_backward_f32_nchw(const LsfaAggArgs* fwd, const LsfaAggGrads* grads, void* stream);

@@ -69,6 +69,7 @@ class LsfaAggGrads(C.Structure):
         ("grad_res", C.c_void_p), ("req_res", C.c_int32),
         ("grad_rnet_w", C.c_void_p), ("grad_rnet_b", C.c_void_p), ("req_rnet", C.c_int32),
         ("workspace", C.c_void_p), ("workspace_bytes", C.c_size_t),
+        ("grad_emb_warp", C.c_void_p), ("grad_emb_cur", C.c_void_p), ("req_emb", C.c_int32),
     ]
 
 
@@ -115,6 +116,8 @@ PROTOTYPES = {
     "lsfa_cosine_logits": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P]),
     "lsfa_cosine_logits_workspace_bytes": (_SZ, [_I, _I, _I, _I, _I]),
     "lsfa_cosine_logits_ws": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _SZ, _P]),
+    "lsfa_cosine_logits_backward_workspace_bytes": (_SZ, [_I, _I, _I, _I]),
+    "lsfa_cosine_logits_backward_f32_nchw": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P, _SZ, _I, _P]),
     "lsfa_unfused_chain_f32_nchw": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),
     "lsfa_unfused_chain_num_launches": (_I, []),
     "lsfa_blend_logits_f32": (_I, [_P, _P, _P, _P, _P, _I, _I, _I, _I, _P]),

@@ -62,11 +62,9 @@ agg_nchw_generic_kernel(const __grid_constant__ AggParams P) {
 
 // ---------------------------------------------------------------------------------------
 // Cosine logits from NCHW embeddings (Fgfa_net compute_weight, SYM:111-116,137-139).
-// Block = 32 pixels x 8 channel groups; each group walks E/8 channels with coalesced
-// 128-byte rows, partial sums are combined in a fixed order in shared memory.
+// Block = 32 pixels x 8 channel groups (cosine_group_sums_nchw); the groups' partial sums are
+// combined in a fixed order in shared memory.
 // ---------------------------------------------------------------------------------------
-constexpr int kCosGroups = 8;
-
 __global__ void __launch_bounds__(32 * kCosGroups)
 cosine_logits_nchw_kernel(const float* __restrict__ ew, const float* __restrict__ ec,
                           float* __restrict__ logits, int E, int HW) {
@@ -75,33 +73,7 @@ cosine_logits_nchw_kernel(const float* __restrict__ ew, const float* __restrict_
   const int lane = threadIdx.x & 31, grp = threadIdx.x >> 5;
   const int p = blockIdx.x * 32 + lane;
   float sww = 0.f, scc = 0.f, swc = 0.f;
-  if (p < HW) {
-    const size_t base = (size_t)n * E * HW + p;
-    const int per = (E + kCosGroups - 1) / kCosGroups;
-    const int e0 = grp * per, e1 = min(E, e0 + per);
-    int e = e0;
-    for (; e + 4 <= e1; e += 4) {
-      float a[4], b[4];
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        a[u] = ldg_stream(ew + base + (size_t)(e + u) * HW);
-        b[u] = ldg_stream(ec + base + (size_t)(e + u) * HW);
-      }
-#pragma unroll
-      for (int u = 0; u < 4; ++u) {
-        sww = fmaf(a[u], a[u], sww);
-        scc = fmaf(b[u], b[u], scc);
-        swc = fmaf(a[u], b[u], swc);
-      }
-    }
-    for (; e < e1; ++e) {
-      const float a = ldg_stream(ew + base + (size_t)e * HW);
-      const float b = ldg_stream(ec + base + (size_t)e * HW);
-      sww = fmaf(a, a, sww);
-      scc = fmaf(b, b, scc);
-      swc = fmaf(a, b, swc);
-    }
-  }
+  if (p < HW) cosine_group_sums_nchw(ew, ec, E, HW, n, p, grp, sww, scc, swc);
   part[0][grp][lane] = sww;
   part[1][grp][lane] = scc;
   part[2][grp][lane] = swc;

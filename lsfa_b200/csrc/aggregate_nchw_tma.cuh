@@ -33,6 +33,12 @@ __device__ __forceinline__ void bulk_s2g(void* dst_gmem, const void* src_smem, u
                "r"(smem_u32(src_smem)), "r"(bytes)
                : "memory");
 }
+// element-wise out += smem (req = kAddTo): one contributor per element, so the result is deterministic
+__device__ __forceinline__ void bulk_reduce_add_s2g(void* dst_gmem, const void* src_smem, uint32_t bytes) {
+  asm volatile("cp.reduce.async.bulk.global.shared::cta.bulk_group.add.f32 [%0], [%1], %2;" ::"l"(dst_gmem),
+               "r"(smem_u32(src_smem)), "r"(bytes)
+               : "memory");
+}
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read_all() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }

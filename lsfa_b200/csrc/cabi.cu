@@ -3,6 +3,7 @@
 // state; errors are reported through a thread-local message like MXGetLastError().
 #include <cmath>
 #include <cstdarg>
+#include <cstddef>
 #include <cstdio>
 #include <cstring>
 
@@ -27,6 +28,10 @@ cudaError_t launch_cosine_logits_nchw(const float* ew, const float* ec, float* l
 size_t cosine_tma_workspace_bytes(int N, int E, int HW);
 cudaError_t launch_cosine_logits_nchw_tma(const float* ew, const float* ec, float* logits, int N, int E, int HW,
                                           void* scratch, size_t scratch_bytes, cudaStream_t st);
+size_t cosine_backward_workspace_bytes(int N, int E, int HW);
+cudaError_t launch_cosine_backward_nchw(const float* ew, const float* ec, const float* gl, const unsigned char* bypass, float* gw,
+                                        float* gc, int add_w, int add_c, int N, int E, int HW, void* workspace,
+                                        size_t workspace_bytes, bool tma_sums, int kernel, cudaStream_t st);
 // aggregate_nhwc.cu
 cudaError_t launch_agg_nhwc(const AggParams& P, bool bf16, int kernel, cudaStream_t st);
 cudaError_t launch_cosine_logits_nhwc(const void* ew, const void* ec, float* logits, int N, int E,
@@ -216,6 +221,15 @@ size_t sched_ws_bytes(const LsfaAggArgs* a) {
   return ((size_t)a->N * parts * sizeof(unsigned) * 3 + 15) / 16 * 16;   // claim counters + 2 row-range words per part
 }
 
+// cosine logits (N,2,H,W) of NCHW embeddings: the all-TMA pre-pass where it serves and `scratch` holds its partial sums
+// (unless tma is false), else the LDG kernel.  The fused forward and the fused backward both compute them here.
+cudaError_t cosine_logits_nchw(const float* ew, const float* ec, float* lg, int N, int E, int HW, void* scratch,
+                               size_t scratch_bytes, bool tma, cudaStream_t st) {
+  cudaError_t ce = cudaErrorNotSupported;
+  if (tma) ce = lsfa::launch_cosine_logits_nchw_tma(ew, ec, lg, N, E, HW, scratch, scratch_bytes, st);
+  if (ce == cudaErrorNotSupported) ce = lsfa::launch_cosine_logits_nchw(ew, ec, lg, N, E, HW, st);
+  return ce;
+}
 int run_aggregate(const LsfaAggArgs* a, void* stream) {
   lsfa::AggParams P;
   int rc = build_params(a, P);
@@ -233,15 +247,11 @@ int run_aggregate(const LsfaAggArgs* a, void* stream) {
       float* lg = static_cast<float*>(a->workspace);
       // with the full workspace: all-TMA pre-pass (deterministic partial sums); else the LDG kernel
       const size_t lg_b = (need + 15) / 16 * 16, part_b = cosine_partials_ws_bytes(a);
-      cudaError_t ce = cudaErrorNotSupported;
-      if (part_b && a->workspace_bytes >= lg_b + part_b && (reinterpret_cast<uintptr_t>(a->workspace) % 16) == 0 &&
-          a->force_generic != 1)
-        ce = lsfa::launch_cosine_logits_nchw_tma(static_cast<const float*>(a->emb_warp), static_cast<const float*>(a->emb_cur),
-                                                 lg, a->N, a->E, P.HW, static_cast<char*>(a->workspace) + lg_b, part_b, st);
-      if (ce == cudaErrorNotSupported)
-        ce = lsfa::launch_cosine_logits_nchw(static_cast<const float*>(a->emb_warp), static_cast<const float*>(a->emb_cur), lg,
-                                             a->N, a->E, P.HW, st);
-      rc = cuda_result(ce, "cosine_logits_nchw launch");
+      const bool tma = part_b && a->workspace_bytes >= lg_b + part_b && (reinterpret_cast<uintptr_t>(a->workspace) % 16) == 0 &&
+                       a->force_generic != 1;
+      rc = cuda_result(cosine_logits_nchw(static_cast<const float*>(a->emb_warp), static_cast<const float*>(a->emb_cur), lg, a->N,
+                                          a->E, P.HW, static_cast<char*>(a->workspace) + lg_b, part_b, tma, st),
+                       "cosine_logits_nchw launch");
       if (rc != LSFA_OK) return rc;
       P.logits = lg;
     }
@@ -481,6 +491,46 @@ int lsfa_cosine_logits_ws(const void* emb_warp, const void* emb_cur, float* logi
     if (e != cudaErrorNotSupported) return cuda_result(e, "cosine_logits_nchw_tma launch");
   }
   return lsfa_cosine_logits(emb_warp, emb_cur, logits, N, E, H, W, layout, stream);
+}
+
+size_t lsfa_cosine_logits_backward_workspace_bytes(int N, int E, int H, int W) {
+  if (N <= 0 || E <= 0 || H <= 0 || W <= 0) return 0;
+  return lsfa::cosine_backward_workspace_bytes(N, E, H * W);
+}
+
+static bool overlaps(const void* p, size_t pb, const void* q, size_t qb) {
+  const uintptr_t a = reinterpret_cast<uintptr_t>(p), b = reinterpret_cast<uintptr_t>(q);
+  return p && q && a < b + qb && b < a + pb;
+}
+
+int lsfa_cosine_logits_backward_f32_nchw(const float* emb_warp, const float* emb_cur, const float* grad_logits,
+                                         float* grad_emb_warp, float* grad_emb_cur, int N, int E, int H, int W, int req_warp,
+                                         int req_cur, void* workspace, size_t workspace_bytes, int kernel, void* stream) {
+  if (!valid_req(req_warp) || !valid_req(req_cur)) return fail(LSFA_E_BADARG, "unknown req %d / %d", req_warp, req_cur);
+  if (kernel < 0 || kernel > 2) return fail(LSFA_E_BADARG, "kernel must be 0 (auto), 1 (plain) or 2 (all-TMA)");
+  if (N <= 0 || E <= 0 || H <= 0 || W <= 0) return fail(LSFA_E_SHAPE, "non-positive dims N=%d E=%d H=%d W=%d", N, E, H, W);
+  if ((long long)H * W >= (1LL << 24)) return fail(LSFA_E_SHAPE, "planes of 2^24 pixels or more are not supported");
+  if (N > 65535) return fail(LSFA_E_SHAPE, "N must be at most 65535");
+  if (req_warp == LSFA_REQ_NULL) grad_emb_warp = nullptr;
+  if (req_cur == LSFA_REQ_NULL) grad_emb_cur = nullptr;
+  if (!grad_emb_warp && !grad_emb_cur) return LSFA_OK;                  // nothing requested
+  if (!emb_warp || !emb_cur || !grad_logits) return fail(LSFA_E_BADARG, "emb_warp, emb_cur and grad_logits are required");
+  const size_t eb = (size_t)N * E * H * W * sizeof(float), lb = (size_t)N * 2 * H * W * sizeof(float);
+  for (const float* gp : {(const float*)grad_emb_warp, (const float*)grad_emb_cur})
+    if (overlaps(gp, eb, emb_warp, eb) || overlaps(gp, eb, emb_cur, eb) || overlaps(gp, eb, grad_logits, lb))
+      return fail(LSFA_E_BADARG, "the gradients must not overlap emb_warp, emb_cur or grad_logits");
+  if (overlaps(grad_emb_warp, eb, grad_emb_cur, eb)) return fail(LSFA_E_BADARG, "grad_emb_warp and grad_emb_cur overlap");
+  const size_t need = lsfa::cosine_backward_workspace_bytes(N, E, H * W);
+  if (!workspace || workspace_bytes < need) return fail(LSFA_E_BADARG, "workspace too small: need %zu bytes", need);
+  if (reinterpret_cast<uintptr_t>(workspace) % 16) return fail(LSFA_E_ALIGN, "workspace must be 16-byte aligned");
+  cudaError_t e = lsfa::launch_cosine_backward_nchw(emb_warp, emb_cur, grad_logits, nullptr, grad_emb_warp, grad_emb_cur,
+                                                    req_warp == LSFA_REQ_ADD, req_cur == LSFA_REQ_ADD, N, E, H * W, workspace,
+                                                    workspace_bytes, true, kernel, as_stream(stream));
+  if (e == cudaErrorNotSupported) {
+    cudaGetLastError();
+    return fail(LSFA_E_UNSUPPORTED, "the all-TMA kernel cannot serve these arguments (plane size, odd E or H*W, alignment)");
+  }
+  return cuda_result(e, "cosine backward launch");
 }
 
 int lsfa_unfused_chain_f32_nchw(const float* key, const float* flow, const float* scale_map, const float* cur,
@@ -774,29 +824,44 @@ int lsfa_nq_logits_bf16_nhwc(const void* x, const void* w1, const float* b1, con
 // ---------------------------------------------------------------------------------------------------------
 namespace {
 struct BwdPlan {
-  bool want_key, want_flow, want_scale, want_cur, want_logits, want_res, want_rnet, want_gw, pool_flow;
-  size_t tail_ws, flow_ws, samp_ws;
+  bool want_key, want_flow, want_scale, want_cur, want_logits, want_res, want_rnet, want_gw, pool_flow, want_emb;
+  size_t tail_ws, flow_ws, samp_ws, cos_ws;
 };
 inline bool wanted(const void* p, int req) { return p != nullptr && req != LSFA_REQ_NULL; }
-int plan_backward(const LsfaAggArgs* a, const LsfaAggGrads* g, BwdPlan& B) {
+// the LsfaAggGrads of binaries built before the embedding gradients existed
+constexpr size_t kAggGradsV1Bytes = offsetof(LsfaAggGrads, grad_emb_warp);
+// COSINE mode: [logits (N,2,H,W)][d/d(logits) (N,2,H,W)][cosine backward scratch], after the other regions
+size_t cosine_bwd_plane_bytes(const LsfaAggArgs* a) { return ((size_t)a->N * 2 * a->H * a->W * 4 + 255) & ~(size_t)255; }
+// Validate fwd and grads; G = *g with the fields an older struct lacks read as NULL / 0.
+int plan_backward(const LsfaAggArgs* a, const LsfaAggGrads* g, BwdPlan& B, LsfaAggGrads& G) {
   if (!a || !g) return fail(LSFA_E_BADARG, "fwd and grads are required");
-  if (g->struct_bytes != (int32_t)sizeof(LsfaAggGrads)) return fail(LSFA_E_BADARG, "grads->struct_bytes=%d, expected %zu", g->struct_bytes, sizeof(LsfaAggGrads));
+  if (g->struct_bytes != (int32_t)sizeof(LsfaAggGrads) && g->struct_bytes != (int32_t)kAggGradsV1Bytes)
+    return fail(LSFA_E_BADARG, "grads->struct_bytes=%d, expected %zu (or %zu without the embedding gradients)", g->struct_bytes,
+                sizeof(LsfaAggGrads), kAggGradsV1Bytes);
+  memset(&G, 0, sizeof(G));
+  memcpy(&G, g, (size_t)g->struct_bytes);
+  g = &G;
   if (a->struct_bytes != (int32_t)sizeof(LsfaAggArgs)) return fail(LSFA_E_BADARG, "fwd->struct_bytes=%d, expected %zu", a->struct_bytes, sizeof(LsfaAggArgs));
   if (a->layout != LSFA_LAYOUT_NCHW_F32) return fail(LSFA_E_UNSUPPORTED, "the backward is built for the NCHW float32 layout");
-  if (a->weight_mode == LSFA_W_COSINE) return fail(LSFA_E_UNSUPPORTED, "LSFA_W_COSINE has no backward (its embeddings are inputs produced outside this library)");
-  const int reqs[7] = {g->req_key, g->req_flow, g->req_scale, g->req_cur, g->req_logits, g->req_res, g->req_rnet};
+  const int reqs[8] = {g->req_key, g->req_flow, g->req_scale, g->req_cur, g->req_logits, g->req_res, g->req_rnet, g->req_emb};
   for (int r : reqs) if (!valid_req(r)) return fail(LSFA_E_BADARG, "unknown req %d", r);
+  const bool cosine = a->weight_mode == LSFA_W_COSINE;
+  B.want_emb = wanted(g->grad_emb_warp, g->req_emb) || wanted(g->grad_emb_cur, g->req_emb);
+  if (B.want_emb && !cosine) return fail(LSFA_E_BADARG, "embedding gradients requested but weight_mode is not COSINE");
+  if (cosine && wanted(g->grad_logits, g->req_logits))
+    return fail(LSFA_E_BADARG, "grad_logits requested in COSINE mode: the logits are computed from the embeddings, not an input");
+  if (cosine && (!a->emb_warp || !a->emb_cur || a->E <= 0)) return fail(LSFA_E_BADARG, "COSINE mode needs emb_warp, emb_cur and E > 0");
   B.want_key = wanted(g->grad_key, g->req_key);
   B.want_flow = wanted(g->grad_flow, g->req_flow);
   B.want_scale = wanted(g->grad_scale, g->req_scale);
   B.want_cur = wanted(g->grad_cur, g->req_cur);
-  B.want_logits = wanted(g->grad_logits, g->req_logits);
+  B.want_logits = wanted(g->grad_logits, g->req_logits) || B.want_emb;   // COSINE: d/d(logits) into the workspace
   B.want_res = wanted(g->grad_res, g->req_res);
   B.want_rnet = wanted(g->grad_rnet_w, g->req_rnet);
   if (B.want_rnet && !g->grad_rnet_b) return fail(LSFA_E_BADARG, "grad_rnet_w and grad_rnet_b go together");
   if (B.want_scale && !a->scale_map) return fail(LSFA_E_BADARG, "grad_scale requested but the forward had no scale_map");
   if (B.want_cur && a->weight_mode == LSFA_W_NONE) return fail(LSFA_E_BADARG, "grad_cur requested but weight_mode is NONE");
-  if (B.want_logits && a->weight_mode != LSFA_W_LOGITS) return fail(LSFA_E_BADARG, "grad_logits requested but weight_mode is not LOGITS");
+  if (B.want_logits && a->weight_mode != LSFA_W_LOGITS && !cosine) return fail(LSFA_E_BADARG, "grad_logits requested but weight_mode is not LOGITS");
   if ((B.want_res || B.want_rnet) && !a->res) return fail(LSFA_E_BADARG, "residual gradients requested but the forward had no res");
   if (B.want_flow && a->flow_kind != LSFA_FLOW_PREPOOLED && a->flow_kind != LSFA_FLOW_GRID)
     return fail(LSFA_E_BADARG, "grad_flow needs LSFA_FLOW_PREPOOLED or LSFA_FLOW_GRID: raw motion vectors are integer data (SYM:319-321)");
@@ -814,40 +879,68 @@ int plan_backward(const LsfaAggArgs* a, const LsfaAggGrads* g, BwdPlan& B) {
   B.flow_ws = B.pool_flow ? (((size_t)a->N * 2 * HW * 4 + 255) & ~(size_t)255) : 0;
   const int Hk = a->key_h > 0 ? a->key_h : a->H, Wk = a->key_w > 0 ? a->key_w : a->W;
   B.samp_ws = B.want_gw ? ((lsfa::bwd_workspace_bytes(a->N, Hk * Wk, HW) + 255) & ~(size_t)255) : 0;
+  B.cos_ws = cosine ? 2 * cosine_bwd_plane_bytes(a) + lsfa::cosine_backward_workspace_bytes(a->N, a->E, HW) : 0;
   return LSFA_OK;
 }
+
 }  // namespace
 
 size_t lsfa_warp_scale_aggregate_backward_workspace_bytes(const LsfaAggArgs* fwd, const LsfaAggGrads* grads) {
   BwdPlan B;
-  if (plan_backward(fwd, grads, B) != LSFA_OK) return 0;
-  return B.tail_ws + B.flow_ws + B.samp_ws;
+  LsfaAggGrads G;
+  if (plan_backward(fwd, grads, B, G) != LSFA_OK) return 0;
+  return B.tail_ws + B.flow_ws + B.samp_ws + B.cos_ws;
 }
 
-int lsfa_warp_scale_aggregate_backward_f32_nchw(const LsfaAggArgs* fwd, const LsfaAggGrads* g, void* stream) {
+int lsfa_warp_scale_aggregate_backward_f32_nchw(const LsfaAggArgs* fwd, const LsfaAggGrads* grads, void* stream) {
   BwdPlan B;
-  if (int r = plan_backward(fwd, g, B)) return r;
+  LsfaAggGrads G;
+  if (int r = plan_backward(fwd, grads, B, G)) return r;
+  const LsfaAggGrads* g = &G;
   if (!g->out_grad) return fail(LSFA_E_BADARG, "out_grad is required");
   lsfa::AggParams P;
   if (int r = build_params(fwd, P)) return r;
   if (P.HWk > 16383) return fail(LSFA_E_UNSUPPORTED, "key planes above 16,383 pixels are not supported by the backward");
-  const size_t need = B.tail_ws + B.flow_ws + B.samp_ws;
+  const size_t need = B.tail_ws + B.flow_ws + B.samp_ws + B.cos_ws;
   if (!g->workspace || g->workspace_bytes < need) return fail(LSFA_E_BADARG, "workspace too small: need %zu bytes", need);
   if (reinterpret_cast<uintptr_t>(g->workspace) & 255) return fail(LSFA_E_ALIGN, "workspace must be 256-byte aligned");
   cudaStream_t st = as_stream(stream);
   char* ws = static_cast<char*>(g->workspace);
+  float* glogits = g->grad_logits;
+  char* cos_ws = ws + B.tail_ws + B.flow_ws + B.samp_ws;
+  const size_t plane_b = fwd->weight_mode == LSFA_W_COSINE ? cosine_bwd_plane_bytes(fwd) : 0;
+  const bool tma_sums = fwd->force_generic != 1;
+  if (fwd->weight_mode == LSFA_W_COSINE) {
+    // the forward's logits, then the LOGITS-mode backward on them with d/d(logits) kept in the workspace
+    float* lg = reinterpret_cast<float*>(cos_ws);
+    glogits = reinterpret_cast<float*>(cos_ws + plane_b);
+    if (int r = cuda_result(cosine_logits_nchw(static_cast<const float*>(fwd->emb_warp), static_cast<const float*>(fwd->emb_cur), lg,
+                                               fwd->N, fwd->E, P.HW, cos_ws + 2 * plane_b, B.cos_ws - 2 * plane_b, tma_sums, st),
+                            "cosine_logits_nchw launch"))
+      return r;
+    P.mode = LSFA_W_LOGITS;
+    P.logits = lg;
+  }
   float* gw = nullptr;
   lsfa::TailBwdRequest R{};
   R.out_grad = g->out_grad;
   R.grad_scale = B.want_scale ? g->grad_scale : nullptr; R.add_scale = g->req_scale == LSFA_REQ_ADD;
   R.grad_cur = B.want_cur ? g->grad_cur : nullptr;       R.add_cur = g->req_cur == LSFA_REQ_ADD;
-  R.grad_logits = B.want_logits ? g->grad_logits : nullptr; R.add_logits = g->req_logits == LSFA_REQ_ADD;
+  R.grad_logits = B.want_logits ? glogits : nullptr;     R.add_logits = B.want_emb ? 0 : g->req_logits == LSFA_REQ_ADD;
   R.grad_res = B.want_res ? g->grad_res : nullptr;       R.add_res = g->req_res == LSFA_REQ_ADD;
   R.grad_rnet_w = B.want_rnet ? g->grad_rnet_w : nullptr; R.grad_rnet_b = B.want_rnet ? g->grad_rnet_b : nullptr;
   R.add_rnet = g->req_rnet == LSFA_REQ_ADD;
   R.want_gw = B.want_gw;
   R.gw_out = &gw;
   if (int r = cuda_result(lsfa::launch_tail_backward(P, R, ws, st), "tail backward launch")) return r;
+  if (B.want_emb) {
+    const bool add = g->req_emb == LSFA_REQ_ADD;
+    if (int r = cuda_result(lsfa::launch_cosine_backward_nchw(static_cast<const float*>(fwd->emb_warp), static_cast<const float*>(fwd->emb_cur),
+                                                              glogits, fwd->bypass, g->grad_emb_warp, g->grad_emb_cur, add, add, fwd->N,
+                                                              fwd->E, P.HW, cos_ws + 2 * plane_b, B.cos_ws - 2 * plane_b, tma_sums, 0, st),
+                            "cosine backward launch"))
+      return r;
+  }
   if (!B.want_gw) return LSFA_OK;
   ws += B.tail_ws;
   const float* coords = static_cast<const float*>(fwd->flow);

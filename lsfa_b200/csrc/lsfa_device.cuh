@@ -548,6 +548,40 @@ __device__ __forceinline__ float ldg_stream(const float* p) {
   asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(v) : "l"(p));
   return v;
 }
+// Per-pixel sums a.a, b.b, a.b of the NCHW cosine (Fgfa_net compute_weight, SYM:111-116): the share of channel
+// group grp (of kCosGroups; E/kCosGroups channels each, coalesced 128-byte rows) for pixel p < HW of frame n.  The
+// caller adds the groups' sums in group order.  The forward (cosine_logits_nchw_kernel) and the backward's coefficient
+// kernel both use it, so the backward recomputes the forward's bits.
+constexpr int kCosGroups = 8;
+__device__ __forceinline__ void cosine_group_sums_nchw(const float* __restrict__ ew, const float* __restrict__ ec, int E, int HW,
+                                                       int n, int p, int grp, float& sww, float& scc, float& swc) {
+  const size_t base = (size_t)n * E * HW + p;
+  const int per = (E + kCosGroups - 1) / kCosGroups;
+  const int e0 = grp * per, e1 = min(E, e0 + per);
+  int e = e0;
+  for (; e + 4 <= e1; e += 4) {
+    float a[4], b[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      a[u] = ldg_stream(ew + base + (size_t)(e + u) * HW);
+      b[u] = ldg_stream(ec + base + (size_t)(e + u) * HW);
+    }
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      sww = fmaf(a[u], a[u], sww);
+      scc = fmaf(b[u], b[u], scc);
+      swc = fmaf(a[u], b[u], swc);
+    }
+  }
+  for (; e < e1; ++e) {
+    const float a = ldg_stream(ew + base + (size_t)e * HW);
+    const float b = ldg_stream(ec + base + (size_t)e * HW);
+    sww = fmaf(a, a, sww);
+    scc = fmaf(b, b, scc);
+    swc = fmaf(a, b, swc);
+  }
+}
+
 // Cache policy of the once-touched streams (compile-time experiment knob):
 //   0: ld.global.nc.L1::no_allocate + st.global.cs   1: ld.global.nc (L1 allocate) + st.global.cs  <- default:
 //      measured 5373 vs 4910 GB/s; the sector a warp shares with its neighbour then hits in L1

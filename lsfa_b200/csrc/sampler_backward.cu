@@ -285,12 +285,6 @@ __global__ void __launch_bounds__(256) bwd_overflow_kernel(const __grid_constant
   }
 }
 
-__device__ __forceinline__ void bulk_reduce_add_s2g(void* dst_gmem, const void* src_smem, uint32_t bytes) {
-  asm volatile("cp.reduce.async.bulk.global.shared::cta.bulk_group.add.f32 [%0], [%1], %2;" ::"l"(dst_gmem),
-               "r"(smem_u32(src_smem)), "r"(bytes)
-               : "memory");
-}
-
 __device__ __forceinline__ void consumer_bar() { asm volatile("bar.sync 1, %0;" ::"n"(kTmaConsumers) : "memory"); }
 
 // ---------------------------------------------------------------------------------------

@@ -28,7 +28,7 @@ __all__ = [
     "GridGenerator", "BilinearSampler", "BilinearSampler_backward", "GridGenerator_backward", "warp_backward",
     "mv_prepare", "mv_pool", "res_pool", "transform_mv_res",
     "sampler_coords", "warp_scale_aggregate", "cur_frame_path", "Nq_aggregate", "Fgfa_aggregate",
-    "mean_aggregate", "blend_logits", "ChooseFeat", "tile_as", "cosine_logits", "unfused_chain", "mv_accumulate", "coviar_residual", "to_nhwc",
+    "mean_aggregate", "blend_logits", "ChooseFeat", "tile_as", "cosine_logits", "cosine_logits_backward", "unfused_chain", "mv_accumulate", "coviar_residual", "to_nhwc",
     "to_nchw", "num_launches",
 ]
 
@@ -536,11 +536,12 @@ class RecordedGraph:
             pass
 
 
-def warp_scale_aggregate_backward(out_grad, key, flow, *, want=("key", "flow", "scale", "cur", "logits", "res", "rnet"), **kw):
-    """Backward of ``warp_scale_aggregate`` (NCHW float32; modes none/add/mean/logits; SYM:306-338 needs it for training):
-    returns a dict of the gradients that exist for these inputs among ``want`` - 'key', 'flow' (prepooled flow or grid
-    only: raw motion vectors are data), 'scale', 'cur', 'logits', 'res', 'rnet_w' + 'rnet_b'.  ``kw`` = the forward's
-    keyword arguments."""
+def warp_scale_aggregate_backward(out_grad, key, flow, *, want=("key", "flow", "scale", "cur", "logits", "res", "rnet", "emb_warp",
+                                                              "emb_cur"), **kw):
+    """Backward of ``warp_scale_aggregate`` (NCHW float32; SYM:306-338 needs it for training): returns a dict of the
+    gradients that exist for these inputs among ``want`` - 'key', 'flow' (prepooled flow or grid only: raw motion vectors
+    are data), 'scale', 'cur', 'logits' (logits mode), 'res', 'rnet_w' + 'rnet_b', 'emb_warp' + 'emb_cur' (cosine mode).
+    ``kw`` = the forward's keyword arguments."""
     import ctypes
     kw = dict(kw)
     kw.pop("out", None)
@@ -568,6 +569,9 @@ def warp_scale_aggregate_backward(out_grad, key, flow, *, want=("key", "flow", "
     g.grad_cur, g.req_cur = mk("cur", kw.get("cur"), kw.get("cur") is not None and mode != "none")
     g.grad_logits, g.req_logits = mk("logits", kw.get("logits"), mode == "logits")
     g.grad_res, g.req_res = mk("res", kw.get("res"), kw.get("res") is not None)
+    g.grad_emb_warp, rw = mk("emb_warp", kw.get("emb_warp"), mode == "cosine")
+    g.grad_emb_cur, rc = mk("emb_cur", kw.get("emb_cur"), mode == "cosine")
+    g.req_emb = max(rw, rc)
     if "rnet" in want and kw.get("res") is not None:
         res["rnet_w"] = torch.empty_like(kw["rnet_w"])
         res["rnet_b"] = torch.empty_like(kw["rnet_b"])
@@ -677,6 +681,44 @@ def cosine_logits(emb_warp, emb_cur, layout="nchw", workspace=None) -> torch.Ten
         A.check(lib.lsfa_cosine_logits_ws(emb_warp.data_ptr(), emb_cur.data_ptr(), logits.data_ptr(), N, E, H, W, lay,
                                           workspace.data_ptr(), workspace.numel() * workspace.element_size(), _stream()))
     return logits
+
+
+_COS_KERNEL = {"auto": 0, "plain": 1, "tma": 2, 0: 0, 1: 1, 2: 2}
+
+
+def cosine_logits_backward(emb_warp, emb_cur, grad_logits, grad_emb_warp=None, grad_emb_cur=None, req_warp="write",
+                           req_cur="write", workspace=None, kernel="auto"):
+    """Backward of ``cosine_logits`` (NCHW float32): from d/d(logits) (N,2,H,W) to (grad_emb_warp, grad_emb_cur), each
+    (N,E,H,W) or None where its req is 'null'.  The logits are recomputed as ``cosine_logits`` computes them with its
+    default workspace.  ``kernel``: 'auto', 'plain' (LDG/STG) or 'tma' (all-TMA; raises where it cannot serve the
+    shape); both give the same bits.  The gradients must not overlap the inputs."""
+    _dev(emb_warp, "emb_warp", torch.float32)
+    _dev(emb_cur, "emb_cur", torch.float32)
+    _dev(grad_logits, "grad_logits", torch.float32)
+    if emb_warp.dim() != 4 or emb_cur.shape != emb_warp.shape:
+        raise ValueError("emb_warp and emb_cur must be (N,E,H,W) of one shape, got %s %s" % (tuple(emb_warp.shape), tuple(emb_cur.shape)))
+    N, E, H, W = emb_warp.shape
+    if tuple(grad_logits.shape) != (N, 2, H, W):
+        raise ValueError("grad_logits must be (N,2,H,W)=%s, got %s" % ((N, 2, H, W), tuple(grad_logits.shape)))
+    grads = []
+    for g, rq, nme in ((grad_emb_warp, _REQ[req_warp], "grad_emb_warp"), (grad_emb_cur, _REQ[req_cur], "grad_emb_cur")):
+        if rq != A.REQ_NULL:
+            if g is None:
+                if rq == A.REQ_ADD:
+                    raise ValueError("req 'add' needs an existing %s" % nme)
+                g = torch.empty_like(emb_warp)
+            _dev(g, nme, torch.float32)
+            if g.shape != emb_warp.shape:
+                raise ValueError("%s must have the embeddings' shape" % nme)
+        grads.append(g if rq != A.REQ_NULL else None)
+    lib = A.load()
+    if workspace is None:
+        workspace = torch.empty(lib.lsfa_cosine_logits_backward_workspace_bytes(N, E, H, W), dtype=torch.uint8, device=emb_warp.device)
+    _dev(workspace, "workspace")
+    A.check(lib.lsfa_cosine_logits_backward_f32_nchw(emb_warp.data_ptr(), emb_cur.data_ptr(), grad_logits.data_ptr(), _ptr(grads[0]),
+                                                     _ptr(grads[1]), N, E, H, W, _REQ[req_warp], _REQ[req_cur], workspace.data_ptr(),
+                                                     workspace.numel() * workspace.element_size(), _COS_KERNEL[kernel], _stream()))
+    return grads[0], grads[1]
 
 
 def unfused_chain(key, flow, scale_map, cur, logits, tmp=None) -> torch.Tensor:

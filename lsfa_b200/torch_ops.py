@@ -10,6 +10,8 @@ the ``lsfa::`` namespace:
     lsfa::mv_pool(mv, im_scale, mode) -> flow
     lsfa::warp_scale_aggregate(key, flow, cur?, scale_map?, logits?, bypass?, weight_mode, flow_kind,
                                im_scale, layout) -> out
+    lsfa::cosine_logits(emb_warp, emb_cur) -> logits      (NCHW float32; Fgfa trains as
+                               warp_scale_aggregate(..., logits=cosine_logits(ew, ec), weight_mode=3))
 
 This is harness only - shapes, dtypes and dispatch; the arithmetic is in liblsfa_b200.so.
 """
@@ -168,3 +170,38 @@ def _wsa_backward(ctx, grad_out):
 
 
 warp_scale_aggregate.register_autograd(_wsa_backward, setup_context=_wsa_setup)
+
+
+# Fgfa_net's weights (SYM:111-116,137-139): the same kernels the fused COSINE mode runs, so that mode trains as
+# warp_scale_aggregate(..., logits=cosine_logits(emb_warp, emb_cur), weight_mode=3)
+@torch.library.custom_op("lsfa::cosine_logits", mutates_args=())
+def cosine_logits(emb_warp: torch.Tensor, emb_cur: torch.Tensor) -> torch.Tensor:
+    return ops.cosine_logits(emb_warp, emb_cur)
+
+
+@cosine_logits.register_fake
+def _(emb_warp, emb_cur):
+    torch._check(emb_warp.dim() == 4 and emb_cur.shape == emb_warp.shape, lambda: "emb_warp, emb_cur (N,E,H,W)")
+    return emb_warp.new_empty((emb_warp.shape[0], 2, emb_warp.shape[2], emb_warp.shape[3]))
+
+
+@torch.library.custom_op("lsfa::cosine_logits_backward", mutates_args=())
+def cosine_logits_backward(emb_warp: torch.Tensor, emb_cur: torch.Tensor, grad_logits: torch.Tensor) -> tuple[torch.Tensor, torch.Tensor]:
+    return ops.cosine_logits_backward(emb_warp, emb_cur, grad_logits.contiguous())
+
+
+@cosine_logits_backward.register_fake
+def _(emb_warp, emb_cur, grad_logits):
+    return torch.empty_like(emb_warp), torch.empty_like(emb_cur)
+
+
+def _cos_setup(ctx, inputs, output):
+    ctx.save_for_backward(*inputs)
+
+
+def _cos_backward(ctx, grad_logits):
+    emb_warp, emb_cur = ctx.saved_tensors
+    return cosine_logits_backward(emb_warp, emb_cur, grad_logits)
+
+
+cosine_logits.register_autograd(_cos_backward, setup_context=_cos_setup)

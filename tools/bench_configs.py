@@ -180,6 +180,54 @@ def cosine_rows(dev, pk, Nc):
         time_ms(lambda: ops.cosine_logits(ew, ec, workspace=wsc)), pk)
 
 
+def cosine_backward_rows(dev):
+    """Backward of the cosine logits, 64 frames x E = 2048 x 38x63, seeded inputs.  Each row is reported as a fraction of
+    the device-to-device copy bandwidth measured here (read + write bytes of a 2 GiB copy), with the card's name and
+    power limit read in the same run."""
+    import subprocess
+    name = torch.cuda.get_device_name(dev)
+    try:
+        power = subprocess.run(["nvidia-smi", "--query-gpu=power.limit", "--format=csv,noheader", "-i", str(dev.index or 0)],
+                               capture_output=True, text=True, timeout=30).stdout.strip()
+    except Exception as e:                         # noqa: BLE001 - reported, not hidden
+        power = "unknown (%s)" % e
+    src = torch.empty(2 << 30, dtype=torch.uint8, device=dev)
+    dst = torch.empty_like(src)
+    copy_ms = time_ms(lambda: dst.copy_(src), 3, 20)
+    copy_gbs = 2 * src.numel() / (copy_ms / 1e3) / 1e9
+    del src, dst
+    print(json.dumps({"config": "device copy (read + write)", "gpu": name, "power_limit": power, "achieved_gbs": round(copy_gbs, 1)}), flush=True)
+    N, C, E, H, W = 64, 1024, 2048, 38, 63
+    HW = H * W
+    g = torch.Generator(device=dev).manual_seed(2)
+    ew = torch.randn((N, E, H, W), device=dev, generator=g)
+    ec = torch.randn((N, E, H, W), device=dev, generator=g)
+    gl = torch.randn((N, 2, H, W), device=dev, generator=g)
+    gw, gc = torch.empty_like(ew), torch.empty_like(ec)
+    ws = torch.empty(ops.A.load().lsfa_cosine_logits_backward_workspace_bytes(N, E, H, W), dtype=torch.uint8, device=dev)
+
+    def out(config, alg, ms, note=""):
+        gbs = N * alg / (ms / 1e3) / 1e9
+        print(json.dumps({"config": config, "frames": N, "ms_per_step": round(ms, 4), "alg_bytes_per_frame": alg, "achieved_gbs": round(gbs, 1),
+                          "frac_of_copy": round(gbs / copy_gbs, 4), "gpu": name, "power_limit": power, "note": note}), flush=True)
+    for kern in ("tma", "plain"):
+        out("cosine logits backward (%s)" % kern, 6 * E * HW * 4 + 8 * HW,
+            time_ms(lambda: ops.cosine_logits_backward(ew, ec, gl, grad_emb_warp=gw, grad_emb_cur=gc, workspace=ws, kernel=kern), 3, 20))
+    out("cosine pre-pass alone (sums + logits, all-TMA)", 2 * E * HW * 4 + 8 * HW,
+        time_ms(lambda: ops.cosine_logits(ew, ec), 3, 20), "the backward's sums pass; the gradient pass is the difference")
+    d = synth(N, C, H, W, 600, 1000, dev)
+    flow = ops.mv_pool(d["mv"])
+    og = torch.randn_like(d["key"])
+    F4 = C * HW * 4
+    out("bwd fused V2 (x scale, logits blend): key, flow, scale, cur, logits", 10 * F4,
+        time_ms(lambda: ops.warp_scale_aggregate_backward(og, d["key"], flow, flow_kind="flow", cur=d["cur"], scale_map=d["scale_map"],
+                                                          weight_mode="logits", logits=d["logits"]), 2, 5))
+    out("bwd fused V3 (x scale, cosine blend): key, flow, scale, cur, emb_warp, emb_cur", 10 * F4 + 6 * E * HW * 4,
+        time_ms(lambda: ops.warp_scale_aggregate_backward(og, d["key"], flow, flow_kind="flow", cur=d["cur"], scale_map=d["scale_map"],
+                                                          weight_mode="cosine", emb_warp=ew, emb_cur=ec), 2, 5),
+        "bytes: the V2 row's + the standalone backward's; the logits are recomputed (another 2 E HW 4)")
+
+
 def nhwc_rows(dev, pk, quick, only_tma=False):
     """Channels-last rows (configs 3 and 4 in bf16, fp32 NHWC, the shipped non-key path and the warp alone in bf16):
     the all-TMA kernel (default), its static batch stride (no claim counter) and the LDG/STG tile kernel."""
@@ -431,9 +479,13 @@ def main():
     ap.add_argument("--only-upstream", action="store_true")
     ap.add_argument("--only-keyframe", action="store_true")
     ap.add_argument("--only-motion", action="store_true")
+    ap.add_argument("--only-cosine-backward", action="store_true")
     args = ap.parse_args()
     dev = torch.device("cuda", 0)
     pk = peak()
+    if args.only_cosine_backward:
+        cosine_backward_rows(dev)
+        return
     if args.only_backward:
         backward_rows(dev, pk, args.quick)
         return
